@@ -5,7 +5,7 @@ Headline metric (BASELINE.json): G1 MSM points/s -- the operation that dominates
 (Poly.BlindEval, algebra.go:348-359) -- on synthetic data: bases k_i*G built on the device, scalars uniform
 below 2^254 (< r).  One "step" = one MSM over the rank's point range.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--log-n L] [--impl reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--log-n L] [--impl reference] [--dump-outputs DIR]
 
 N = 1: one MSM of 2^L points (default L = 24, configs[3] of BASELINE.json, the size the north-star's roofline
 target is quoted on).  N > 1 (torchrun, one rank per GPU): every rank owns its own 2^L-point range (weak
@@ -24,6 +24,9 @@ Secondary sections of the same JSON line (all of BASELINE.json's configs):
   cpu_baseline  the reference's algorithms restated in C (oracle/), timed on this box's host cores: BlindEval rate
                 and the WHOLE reference flow (ToQAP -> setup -> Groth16Prove) at the sizes where it finishes
 `--impl reference` times that CPU restatement of BlindEval on all host threads on a bounded sample.
+`--dump-outputs DIR` writes the headline's result from its last timed step to DIR/g1_msm_point.npy: the compressed
+point (summed over the ranks with N > 1) as its 48 byte values in float64.  The inputs are seeded, so two builds
+run with the same arguments can be compared file for file.
 """
 from __future__ import annotations
 
@@ -262,7 +265,11 @@ def main():
     ap.add_argument("--phgr13-log-n", default="16,20", help="PHGR13 prove sizes (one GPU; '' = skip)")
     ap.add_argument("--cpu-budget-s", type=float, default=30.0, help="time budget of the CPU Groth16 flow")
     ap.add_argument("--watchdog-s", type=float, default=900.0, help="print the line as far as it got after this many seconds")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the headline MSM's result of the last timed step to DIR/g1_msm_point.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.warmup < 3 and args.impl != "reference":
         args.warmup = 3
     if args.impl == "reference":
@@ -371,6 +378,11 @@ def main():
     for k in phase:
         phase[k] = tm[k]
     clocks = sampler.stop() if sampler else None
+    if args.dump_outputs and rank == 0:
+        # before the e2e steps, which reuse d_part with several ranks; d_all holds the last step's gathered partials
+        be._check(lib.ps_msm_combine(be.ctx, L.PS_G1, C.c_void_p((d_all if world > 1 else d_part).data_ptr()), world, out))
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "g1_msm_point.npy"), np.frombuffer(out.raw, dtype=np.uint8).astype(np.float64))
 
     # e2e: host buffers in, host bytes out, copies inside the timed region
     progress("G1 e2e")
