@@ -109,6 +109,41 @@ def build_variant(name: str, flags, tus=("capi_poly.cu",)) -> str:
     return out
 
 
+TEST_BUILD = os.path.join(ROOT, "tests", "_build")
+DEVICE_HARNESS = os.path.join(ROOT, "tests", "device_arith.cu")
+
+
+def can_write(dir_path: str) -> bool:
+    """dir_path exists and is writable, or can be created"""
+    while not os.path.isdir(dir_path):
+        parent = os.path.dirname(dir_path)
+        if parent == dir_path:
+            return False
+        dir_path = parent
+    return os.access(dir_path, os.W_OK | os.X_OK)
+
+
+def build_device_harness(out_dir: str = TEST_BUILD) -> str:
+    """TEST-ONLY: the field / group-law harness of the GPU suite (tests/device_arith.cu, loaded by
+    tests/test_gpu_arith.py) as out_dir/libdevice_arith.so for sm_100a, rebuilt when it or a header it includes
+    has changed.  Written under a temporary name and renamed, so a reader never loads a partial file."""
+    so = os.path.join(out_dir, "libdevice_arith.so")
+    if not stale(so, _deps(DEVICE_HARNESS)):
+        return so
+    os.makedirs(out_dir, exist_ok=True)
+    tmp = "%s.%d.tmp" % (so, os.getpid())
+    nvcc = os.environ.get("NVCC", "nvcc")
+    cmd = [nvcc] + NVCC_FLAGS + ["-split-compile", "0", "-shared", "-o", tmp, DEVICE_HARNESS]
+    print("[playsnark_b200] " + " ".join(cmd), file=sys.stderr)
+    try:
+        subprocess.check_call(cmd, cwd=ROOT)
+        os.replace(tmp, so)
+    finally:
+        if os.path.exists(tmp):
+            os.remove(tmp)
+    return so
+
+
 def build_host_emulation(out_dir: str) -> str:
     """TEST-ONLY: the same sources with -DPS_HOST_EMU (kernel bodies driven by serial loops)."""
     os.makedirs(out_dir, exist_ok=True)
