@@ -254,6 +254,27 @@ int ps_pairing_check_batch(ps_ctx* ctx, const uint8_t* g1_points, const uint8_t*
 int ps_g16_verify(ps_ctx* ctx, const uint8_t* alpha, const uint8_t* beta2, const uint8_t* gamma2, const uint8_t* delta2,
                   const uint8_t* iolp, size_t n_io, const uint8_t* io_be, const uint8_t* A, const uint8_t* B,
                   const uint8_t* C, int* ok);
+/* Groth16Verify for n_proofs proofs against one key as ONE combined pairing-product check with random 128-bit weights
+ * rho_i:  prod_i e(-rho_i A_i, B_i) e(S Alpha, Beta2) e(L, Gamma) e(Cs, Delta2) == 1  with S = sum rho_i,
+ * L = sum_j (sum_i rho_i io_i[j]) IoLP_j (one MSM), Cs = sum rho_i C_i: n_proofs + 3 Miller loops, one final exponentiation.
+ * A batch of valid proofs is accepted; one with an invalid proof is rejected except with probability <= 2^-128 over the
+ * weights, which must therefore be unpredictable to whoever made the proofs.
+ *   io_be: n_proofs x n_io x 32 bytes, proof-major.  A / B / C: n_proofs compressed points each (48 / 96 / 48 B).
+ *   weights: NULL (drawn by the library from the operating system: getrandom) or n_proofs x 16 bytes big-endian (tests).
+ *   *ok = 1 iff every proof verifies.  per_proof: NULL, or n_proofs bytes, 1 = that proof verifies (on a failed batch the
+ *   library bisects over a binary tree of the proofs: O(k log n_proofs) node checks for k invalid proofs).
+ * Status:
+ *   - a key point that does not decode (curve; subgroup when the "subgroup_check" option is set): PS_ERR_ENCODING;
+ *     an io value >= r: PS_ERR_ENCODING;
+ *   - a proof point that does not decode or lies outside the prime-order subgroup (always checked, whatever
+ *     "subgroup_check" says): that proof is invalid (per_proof[i] = 0, *ok = 0) and left out of the combined sums; the
+ *     call returns PS_OK and decides the other proofs;
+ *   - a weight of zero: PS_ERR_ARG;  n_proofs == 0: *ok = 1, nothing launched;
+ *   - n_proofs > 2^20, or n_proofs * n_io >= 2^31: PS_ERR_UNSUPPORTED.                                                */
+int ps_g16_verify_batch(ps_ctx* ctx, const uint8_t* alpha, const uint8_t* beta2, const uint8_t* gamma2,
+                        const uint8_t* delta2, const uint8_t* iolp, size_t n_io, size_t n_proofs, const uint8_t* io_be,
+                        const uint8_t* A, const uint8_t* B, const uint8_t* C, const uint8_t* weights,
+                        int* ok, uint8_t* per_proof);
 /* PHGR13Verify (pinochio.go:281-375): division check, three CRS checks, linear check.  vk_fixed = the 576 bytes of
  * ps_phgr13_setup; vs / ws / ys = the commitments of the first n_io (public) variables (48 / 96 / 48 B each);
  * proof = the 432 bytes of ps_phgr13_prove.                                                                     */
@@ -325,6 +346,10 @@ int ps_last_msm_timing(ps_ctx* ctx, float out_ms[5]);
  * [1] MSMs A and C (G1, one batched pipeline), [2] 0 (kept for layout), [3] normalise + encode A and C, [4] what
  * then remains of MSM B and its encoding (G2, concurrently on a second stream), [5] total          */
 int ps_last_prove_timing(ps_ctx* ctx, float out_ms[6]);
+/* device time in ms of the last ps_g16_verify_batch, by phase: [0] upload of points and weights, [1] decode + subgroup
+ * checks, [2] weighting (rho_i A_i, rho_i C_i), [3] upload + conversion of the io values, [4] the proofs' Miller loops, [5] tree of products and sums, [6] root check
+ * (io sums + MSM, three Miller loops, final exponentiation), [7] bisection for the per-proof verdicts, [8] total      */
+int ps_last_verify_batch_timing(ps_ctx* ctx, float out_ms[9]);
 
 #ifdef __cplusplus
 }

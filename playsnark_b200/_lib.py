@@ -72,6 +72,7 @@ SYMBOLS = [
     ("ps_phgr13_prove", _I, [_P, _P, _P, _P, _P, _P]),
     ("ps_pairing_check_batch", _I, [_P, _B, _B, C.POINTER(C.c_uint32), _SZ, _I, _P]),
     ("ps_g16_verify", _I, [_P, _B, _B, _B, _B, _B, _SZ, _B, _B, _B, _B, C.POINTER(C.c_int)]),
+    ("ps_g16_verify_batch", _I, [_P, _B, _B, _B, _B, _B, _SZ, _SZ, _P, _P, _P, _P, _P, C.POINTER(C.c_int), _P]),
     ("ps_phgr13_verify", _I, [_P, _B, _B, _B, _B, _SZ, _B, _B, C.POINTER(C.c_int)]),
     ("ps_mctx_create", _I, [C.POINTER(C.c_int), _I, C.POINTER(_P)]),
     ("ps_mctx_destroy", None, [_P]),
@@ -94,6 +95,7 @@ SYMBOLS = [
     ("ps_bench_fieldmul", _I, [_P, _I, _I, C.POINTER(C.c_double), C.POINTER(C.c_double)]),
     ("ps_last_msm_timing", _I, [_P, C.POINTER(C.c_float)]),
     ("ps_last_prove_timing", _I, [_P, C.POINTER(C.c_float)]),
+    ("ps_last_verify_batch_timing", _I, [_P, C.POINTER(C.c_float)]),
 ]
 
 

@@ -778,6 +778,51 @@ def Groth16Verify(tr: Groth16Setup, q, p: "Groth16Proof", io: Vector, backend: O
     return ok.value == 1
 
 
+def Groth16VerifyBatch(tr: Groth16Setup, q, proofs: Sequence["Groth16Proof"], ios, backend: Optional[Backend] = None,
+                       weights: Optional[Sequence[int]] = None, per_proof: bool = False):
+    """Groth16Verify for many proofs against one key, decided as ONE combined pairing-product check with random 128-bit
+    weights (ps_g16_verify_batch).  `ios` = one public-input vector per proof (each at least as long as IoLP, like
+    Groth16Verify's `io`), or one wire-format blob / HostBuffer of len(proofs) x len(IoLP) values, proof-major.
+    `weights` (tests only) = one nonzero integer below 2^128 per proof; by default the library draws them from the
+    operating system.  Returns True iff every proof verifies; with per_proof=True a list with one verdict per proof.
+    A proof whose points do not decode, or lie outside the prime-order subgroup, is simply invalid."""
+    b = backend or default_backend()
+    if tr.fmt != L.PS_FMT_COMPRESSED:
+        raise ValueError("Groth16VerifyBatch takes the setup's points in compressed form (fmt = PS_FMT_COMPRESSED)")
+    n_io, n = len(tr.IoLP), len(proofs)
+    if isinstance(ios, (HostBuffer, bytes, bytearray, memoryview)):
+        nbytes = ios.nbytes if isinstance(ios, HostBuffer) else len(ios)
+        if nbytes != n * n_io * 32:
+            raise ValueError("different number of public inputs than IoLP elements")
+        io_arg = _fr_bytes(ios)
+    else:
+        if len(ios) != n:
+            raise ValueError("different number of proofs than public input vectors")
+        for io in ios:
+            if len(io) < n_io:
+                raise ValueError("different number of public inputs than IoLP elements")
+        io_arg = b"".join(_fr_bytes(list(io[:n_io])) for io in ios)
+    w_arg = None
+    if weights is not None:
+        if len(weights) != n:
+            raise ValueError("one weight per proof")
+        if any(not 0 < int(w) < 1 << 128 for w in weights):
+            raise ValueError("weights must be nonzero 128-bit integers")
+        w_arg = b"".join(int(w).to_bytes(16, "big") for w in weights)
+    ok = C.c_int(0)
+    verdicts = C.create_string_buffer(max(1, n)) if per_proof else None
+    st = b.lib.ps_g16_verify_batch(b.ctx, _join(tr.Alpha), _join(tr.Beta2), tr.Gamma, _join(tr.Delta2), b"".join(tr.IoLP) or b"\0",
+                                   n_io, n, io_arg or None, b"".join(p.A for p in proofs) or None,
+                                   b"".join(p.B for p in proofs) or None, b"".join(p.C for p in proofs) or None, w_arg,
+                                   C.byref(ok), verdicts)
+    if st == L.PS_ERR_ARG and weights is not None:
+        raise ValueError("weights must be nonzero 128-bit integers")
+    b._check(st)
+    if per_proof:
+        return [verdicts.raw[i] == 1 for i in range(n)]
+    return ok.value == 1
+
+
 def PHGR13Verify(vk: dict, qap, p: PHGR13Proof, io: Vector, backend: Optional[Backend] = None) -> bool:
     """PHGR13Verify, pinochio.go:281-375.  `vk` = the dict NewPHGR13TrustedSetup(..., with_vk=True) returns (av, aw, ay,
     gamma, bgamma, bgamma2, yts and the per-variable commitments vs / ws / ys); `io` = the first nbVars - nbIO values of

@@ -262,6 +262,20 @@ int phgr13_key_alloc(ps_ctx* ctx, ps_phgr13_key* k, size_t n_gates, size_t n_mid
 
 }  // namespace
 
+namespace ps {
+int msm_rows_g1(ps_ctx* ctx, const ps_bases* b, const uint32_t* d_scalars, size_t rows, int mont, void* d_out_xyzz) {
+  if (!b || b->group != PS_G1) return PS_ERR_ARG;
+  G1XYZZ* out = (G1XYZZ*)d_out_xyzz;
+  for (size_t r0 = 0; r0 < rows; r0 += MSM_MAX_SEG) {
+    const int cnt = (int)(rows - r0 < (size_t)MSM_MAX_SEG ? rows - r0 : (size_t)MSM_MAX_SEG);
+    SegSpec sg[MSM_MAX_SEG];
+    for (int k = 0; k < cnt; k++) sg[k] = SegSpec{b, 0, d_scalars + (r0 + k) * b->n * 8, b->n, mont, k};
+    PS_TRY(msm_batch<Fp>(ctx, sg, cnt, cnt, out + r0));
+  }
+  return PS_OK;
+}
+}  // namespace ps
+
 extern "C" {
 
 const char* ps_strerror(int status) {
@@ -326,6 +340,7 @@ int ps_ctx_create(int device, ps_ctx** out) {
     PS_CUDA_TRY(cudaEventCreateWithFlags(&e, cudaEventDisableTiming)); ctx->ev_join = e;
     for (int i = 0; i < 5; i++) { PS_CUDA_TRY(cudaEventCreate(&e)); ctx->ev[i] = e; }
     for (int i = 0; i < 6; i++) { PS_CUDA_TRY(cudaEventCreate(&e)); ctx->evp[i] = e; }
+    for (int i = 0; i < 9; i++) { PS_CUDA_TRY(cudaEventCreate(&e)); ctx->evv[i] = e; }
     return PS_OK;
   };
   rc = init();
@@ -411,6 +426,7 @@ void ps_ctx_destroy(ps_ctx* ctx) {
 #if PS_GPU
   for (int i = 0; i < 5; i++) if (ctx->ev[i]) cudaEventDestroy((cudaEvent_t)ctx->ev[i]);
   for (int i = 0; i < 6; i++) if (ctx->evp[i]) cudaEventDestroy((cudaEvent_t)ctx->evp[i]);
+  for (int i = 0; i < 9; i++) if (ctx->evv[i]) cudaEventDestroy((cudaEvent_t)ctx->evv[i]);
   if (ctx->own_stream && ctx->stream) cudaStreamDestroy(ctx->stream);
   if (ctx->stream2) cudaStreamDestroy(ctx->stream2);
   if (ctx->ev_fork) cudaEventDestroy((cudaEvent_t)ctx->ev_fork);
@@ -554,6 +570,19 @@ int ps_last_prove_timing(ps_ctx* ctx, float out_ms[6]) {
   for (int i = 0; i < 5; i++)
     PS_CUDA_TRY(cudaEventElapsedTime(&out_ms[i], (cudaEvent_t)ctx->evp[i], (cudaEvent_t)ctx->evp[i + 1]));
   PS_CUDA_TRY(cudaEventElapsedTime(&out_ms[5], (cudaEvent_t)ctx->evp[0], (cudaEvent_t)ctx->evp[5]));
+#endif
+  return PS_OK;
+}
+
+int ps_last_verify_batch_timing(ps_ctx* ctx, float out_ms[9]) {
+  if (!ctx || !out_ms) return PS_ERR_ARG;
+  for (int i = 0; i < 9; i++) out_ms[i] = 0.f;
+#if PS_GPU
+  if (!ctx->evv_valid) return PS_ERR_ARG;
+  PS_CUDA_TRY(cudaEventSynchronize((cudaEvent_t)ctx->evv[8]));
+  for (int i = 0; i < 8; i++)
+    PS_CUDA_TRY(cudaEventElapsedTime(&out_ms[i], (cudaEvent_t)ctx->evv[i], (cudaEvent_t)ctx->evv[i + 1]));
+  PS_CUDA_TRY(cudaEventElapsedTime(&out_ms[8], (cudaEvent_t)ctx->evv[0], (cudaEvent_t)ctx->evv[8]));
 #endif
   return PS_OK;
 }

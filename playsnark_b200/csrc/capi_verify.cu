@@ -9,7 +9,10 @@
 #include "group_ops.cuh"
 #include "pairing.cuh"
 #include "poly_api.cuh"
+#include "verify_batch.cuh"
 
+#include <errno.h>
+#include <sys/random.h>
 #include <vector>
 
 using namespace ps;
@@ -63,6 +66,67 @@ int g2_generator_bytes(ps_ctx* ctx, uint8_t out[96]) {
   ps_bases_free(b);
   return rc;
 }
+
+// largest batch of ps_g16_verify_batch: the per-proof device state of 2^20 proofs (tree nodes, points, Miller values) is about 3 GB
+constexpr size_t VERIFY_BATCH_MAX = size_t(1) << 20;
+
+// n nonzero 128-bit weights from the operating system's generator, as 4 little-endian limbs each
+int draw_weights(size_t n, std::vector<uint32_t>& limbs) {
+  for (size_t i = 0; i < n; i++) {
+    uint32_t* k = limbs.data() + 4 * i;
+    do {
+      size_t got = 0;
+      while (got < 16) {
+        ssize_t r = getrandom((uint8_t*)k + got, 16 - got, 0);
+        if (r < 0 && errno == EINTR) continue;
+        if (r <= 0) return PS_ERR_UNSUPPORTED;
+        got += (size_t)r;
+      }
+    } while ((k[0] | k[1] | k[2] | k[3]) == 0);
+  }
+  return PS_OK;
+}
+
+// Device state of one ps_g16_verify_batch call (arena memory); check_nodes runs the node check of the listed nodes
+struct VbState {
+  ps_ctx* ctx;
+  const ps_bases* iolp;    // null when n_io == 0
+  uint32_t n, P, n_io;
+  const Fr* io;            // n x n_io, Montgomery
+  const Fr* w;             // per-proof weights (0 for a proof that did not decode)
+  Fp12* f; G1XYZZ* cs; Fr* s;
+  Fp12* fe; uint8_t* bad;  // per node: value after the final exponentiation, check failed
+  const G1Affine* alpha; const G2Affine* key2;
+
+  int check_nodes(const std::vector<uint32_t>& nodes) {
+    const size_t m = nodes.size();
+    Arena& ar = ctx->arena;
+    ps_stream_t st = ctx->stream;
+    uint32_t* d_nodes = ar.take<uint32_t>(m);
+    G1XYZZ* L = ar.take<G1XYZZ>(m);
+    G1XYZZ* p = ar.take<G1XYZZ>(3 * m);
+    G1Affine* pa = ar.take<G1Affine>(3 * m);
+    G2Affine* q = ar.take<G2Affine>(3 * m);
+    Fp12* fm = ar.take<Fp12>(3 * m);
+    Fp12* acc = ar.take<Fp12>(m);
+    Fr* sc = n_io ? ar.take<Fr>(m * n_io) : nullptr;
+    if (!d_nodes || !L || !p || !pa || !q || !fm || !acc || (n_io && !sc)) return PS_ERR_ALLOC;
+    PS_TRY(dev_h2d(d_nodes, nodes.data(), m * 4, st));
+    if (n_io) {
+      PS_LAUNCH(VbIoCombineK, st, m * n_io, n_io, P, n, (const uint32_t*)d_nodes, io, w, sc);
+      PS_TRY(msm_rows_g1(ctx, iolp, (const uint32_t*)sc, m, 0, L));
+    } else {
+      PS_TRY(dev_memset(L, 0, m * sizeof(G1XYZZ), st));
+    }
+    PS_LAUNCH(VbNodePointsK, st, m, (const uint32_t*)d_nodes, (const Fr*)s, (const G1XYZZ*)cs, (const G1XYZZ*)L, alpha, key2, p, q);
+    PS_TRY(GroupOps<Fp>::to_affine(ctx, p, 3 * m, pa));
+    PS_LAUNCH(PairingMillerK, st, 3 * m, (const G1Affine*)pa, (const G2Affine*)q, fm);
+    PS_LAUNCH(VbNodeProductK, st, m, (const uint32_t*)d_nodes, (const Fp12*)f, (const Fp12*)fm, acc);
+    PS_LAUNCH(VbFinalExpK, st, m, (const Fp12*)acc, fm);                   // the Miller values are consumed: reuse fm[0, m)
+    PS_LAUNCH(VbVerdictK, st, m, (const uint32_t*)d_nodes, (const Fp12*)fm, fe, bad);
+    return PS_OK;
+  }
+};
 
 }  // namespace
 
@@ -130,6 +194,137 @@ int ps_g16_verify(ps_ctx* ctx, const uint8_t* alpha, const uint8_t* beta2, const
   uint8_t res = 0;
   PS_TRY(ps_pairing_check_batch(ctx, g1, g2, &count, 1, PS_FMT_COMPRESSED, &res));
   *ok = res ? 1 : 0;
+  return PS_OK;
+}
+
+int ps_g16_verify_batch(ps_ctx* ctx, const uint8_t* alpha, const uint8_t* beta2, const uint8_t* gamma2, const uint8_t* delta2,
+                        const uint8_t* iolp, size_t n_io, size_t n_proofs, const uint8_t* io_be, const uint8_t* A, const uint8_t* B,
+                        const uint8_t* C, const uint8_t* weights, int* ok, uint8_t* per_proof) {
+  if (!ctx || !alpha || !beta2 || !gamma2 || !delta2 || !ok || (n_io && !iolp)) return PS_ERR_ARG;
+  if (n_proofs && (!A || !B || !C || (n_io && !io_be))) return PS_ERR_ARG;
+  *ok = 0;
+  if (n_proofs > VERIFY_BATCH_MAX || n_io > (1u << 26) || (unsigned long long)n_proofs * n_io >= (1ull << 31))
+    return PS_ERR_UNSUPPORTED;
+  std::vector<uint32_t> rho(4 * n_proofs);
+  if (weights) {
+    for (size_t i = 0; i < n_proofs; i++) {
+      const uint8_t* b = weights + 16 * i;
+      uint32_t* k = rho.data() + 4 * i;
+      for (int j = 0; j < 4; j++)
+        k[j] = ((uint32_t)b[12 - 4 * j] << 24) | ((uint32_t)b[13 - 4 * j] << 16) | ((uint32_t)b[14 - 4 * j] << 8) | b[15 - 4 * j];
+      if ((k[0] | k[1] | k[2] | k[3]) == 0) return PS_ERR_ARG;
+    }
+  }
+  if (n_proofs == 0) { *ok = 1; return PS_OK; }
+  if (!weights) PS_TRY(draw_weights(n_proofs, rho));
+  // the key's IoLP as a base set: decoding errors of key points are the caller's (PS_ERR_ENCODING)
+  ps_bases* bl = nullptr;
+  if (n_io) PS_TRY(ps_bases_load(ctx, PS_G1, iolp, n_io, PS_FMT_COMPRESSED, 0, 1, &bl));
+  struct Free { ps_bases* b; ~Free() { ps_bases_free(b); } } free_bl{bl};
+  PS_TRY(begin_call(ctx));
+  ctx->evv_valid = false;
+  ps_stream_t st = ctx->stream;
+  Arena& ar = ctx->arena;
+  const uint32_t n = (uint32_t)n_proofs;
+  uint32_t P = 1;
+  while (P < n) P <<= 1;
+  uint8_t* d_key = ar.take<uint8_t>(48 + 3 * 96);
+  uint8_t* d_pts = ar.take<uint8_t>(n_proofs * (48 + 96 + 48));
+  uint32_t* d_rho = ar.take<uint32_t>(4 * n_proofs);
+  G1Affine* d_alpha = ar.take<G1Affine>(1);
+  G2Affine* d_key2 = ar.take<G2Affine>(3);
+  G1Affine* d_A = ar.take<G1Affine>(n);
+  G1Affine* d_C = ar.take<G1Affine>(n);
+  G2Affine* d_B = ar.take<G2Affine>(P);
+  uint8_t* d_st = ar.take<uint8_t>(3 * n_proofs);
+  Fr* d_w = ar.take<Fr>(n);
+  uint8_t* d_valid = ar.take<uint8_t>(n);
+  G1XYZZ* d_negA = ar.take<G1XYZZ>(P);
+  G1Affine* d_negAa = ar.take<G1Affine>(P);
+  Fp12* d_f = ar.take<Fp12>(2 * P);
+  G1XYZZ* d_cs = ar.take<G1XYZZ>(2 * P);
+  Fr* d_s = ar.take<Fr>(2 * P);
+  Fp12* d_fe = ar.take<Fp12>(2 * P);
+  uint8_t* d_bad = ar.take<uint8_t>(2 * P);
+  uint32_t* d_err = ar.take<uint32_t>(1);   // key points; proof points report per proof
+  if (!d_key || !d_pts || !d_rho || !d_alpha || !d_key2 || !d_A || !d_C || !d_B || !d_st || !d_w ||
+      !d_valid || !d_negA || !d_negAa || !d_f || !d_cs || !d_s || !d_fe || !d_bad || !d_err)
+    return PS_ERR_ALLOC;
+  PS_TRY(ctx_verify_event(ctx, 0));
+  std::vector<uint8_t> key(48 + 3 * 96);
+  memcpy(key.data(), alpha, 48); memcpy(key.data() + 48, beta2, 96); memcpy(key.data() + 144, gamma2, 96);
+  memcpy(key.data() + 240, delta2, 96);
+  PS_TRY(dev_h2d(d_key, key.data(), key.size(), st));
+  PS_TRY(dev_h2d(d_pts, A, n_proofs * 48, st));
+  PS_TRY(dev_h2d(d_pts + n_proofs * 48, C, n_proofs * 48, st));
+  PS_TRY(dev_h2d(d_pts + n_proofs * 96, B, n_proofs * 96, st));
+  PS_TRY(dev_h2d(d_rho, rho.data(), rho.size() * 4, st));
+  PS_TRY(dev_memset(d_err, 0, 4, st));
+  PS_TRY(dev_memset(d_bad, 0, 2 * P, st));
+  if (P > n) PS_TRY(dev_memset(d_B + n, 0, (P - n) * sizeof(G2Affine), st));   // empty slots pair with infinity
+  PS_TRY(ctx_verify_event(ctx, 1));
+  // key points follow the context's subgroup_check; proof points are untrusted and always checked, with a status each
+  const bool sub = ctx->subgroup_check != 0;
+  PS_TRY(GroupOps<Fp>::decode(ctx, d_key, 1, PS_FMT_COMPRESSED, d_alpha, d_err, sub));
+  PS_TRY(GroupOps<Fp2>::decode(ctx, d_key + 48, 3, PS_FMT_COMPRESSED, d_key2, d_err, sub));
+  uint32_t* d_perr = ar.take<uint32_t>(1);
+  if (!d_perr) return PS_ERR_ALLOC;
+  PS_TRY(GroupOps<Fp>::decode(ctx, d_pts, n, PS_FMT_COMPRESSED, d_A, d_perr, true, d_st));
+  PS_TRY(GroupOps<Fp2>::decode(ctx, d_pts + n_proofs * 96, n, PS_FMT_COMPRESSED, d_B, d_perr, true, d_st + n_proofs));
+  PS_TRY(GroupOps<Fp>::decode(ctx, d_pts + n_proofs * 48, n, PS_FMT_COMPRESSED, d_C, d_perr, true, d_st + 2 * n_proofs));
+  PS_TRY(ctx_verify_event(ctx, 2));
+  PS_LAUNCH(VbWeighK, st, P, n, P, (const uint32_t*)d_rho, (const uint8_t*)d_st, (const G1Affine*)d_A, (const G1Affine*)d_C, d_negA, d_cs,
+            d_s, d_w, d_valid);
+  PS_TRY(GroupOps<Fp>::to_affine(ctx, d_negA, P, d_negAa));
+  PS_TRY(ctx_verify_event(ctx, 3));
+  uint32_t *d_io = nullptr, *d_ioerr = nullptr;
+  if (n_io) PS_TRY(stage_scalars(ctx, io_be, n_proofs * n_io, 1, &d_io, &d_ioerr));
+  VbState vs{ctx, bl, n, P, (uint32_t)n_io, (const Fr*)d_io, d_w, d_f, d_cs, d_s, d_fe, d_bad, d_alpha, d_key2};
+  PS_TRY(ctx_verify_event(ctx, 4));   // the io sums of the root run inside its node check (phase 6)
+  PS_LAUNCH(PairingMillerK, st, P, (const G1Affine*)d_negAa, (const G2Affine*)d_B, d_f + P);
+  PS_TRY(ctx_verify_event(ctx, 5));
+  for (uint32_t first = P >> 1; first >= 1; first >>= 1) PS_LAUNCH(VbTreeLevelK, st, first, first, d_f, d_cs, d_s);
+  PS_TRY(ctx_verify_event(ctx, 6));
+  PS_TRY(vs.check_nodes(std::vector<uint32_t>{1}));
+  PS_TRY(ctx_verify_event(ctx, 7));
+  std::vector<uint8_t> valid(n_proofs);
+  uint8_t root_bad = 0;
+  PS_TRY(dev_d2h(valid.data(), d_valid, n_proofs, st));
+  PS_TRY(dev_d2h(&root_bad, d_bad + 1, 1, st));
+  uint32_t herr[2] = {0, 0};
+  PS_TRY(dev_d2h(herr, d_err, 4, st));
+  if (n_io) PS_TRY(dev_d2h(herr + 1, d_ioerr, 4, st));
+  PS_TRY(dev_sync(st));
+  if (herr[0] || herr[1]) return PS_ERR_ENCODING;
+  bool all_valid = true;
+  for (size_t i = 0; i < n_proofs; i++) all_valid = all_valid && valid[i];
+  *ok = (all_valid && !root_bad) ? 1 : 0;
+  if (per_proof) {
+    memcpy(per_proof, valid.data(), n_proofs);
+    // bisection: level by level, only below failing nodes; one node check per failing node (its left child)
+    std::vector<uint32_t> failing;
+    if (root_bad) failing.push_back(1);
+    std::vector<uint8_t> hbad;
+    while (!failing.empty() && failing[0] < P) {
+      std::vector<uint32_t> lefts(failing.size());
+      for (size_t t = 0; t < failing.size(); t++) lefts[t] = 2 * failing[t];
+      PS_TRY(vs.check_nodes(lefts));
+      uint32_t level_first = 1;
+      while (level_first * 2 <= lefts[0]) level_first <<= 1;   // first node of the children's level
+      hbad.resize(level_first);
+      PS_TRY(dev_d2h(hbad.data(), d_bad + level_first, level_first, st));
+      PS_TRY(dev_sync(st));
+      std::vector<uint32_t> next;
+      for (uint32_t k : lefts)
+        for (uint32_t c = k; c <= k + 1; c++)
+          if (hbad[c - level_first]) next.push_back(c);
+      failing.swap(next);
+    }
+    for (uint32_t k : failing)
+      if (k >= P && k - P < n) per_proof[k - P] = 0;
+  }
+  PS_TRY(ctx_verify_event(ctx, 8));
+  ctx->evv_valid = true;
   return PS_OK;
 }
 

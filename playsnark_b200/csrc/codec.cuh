@@ -140,9 +140,11 @@ PS_DEV bool inf_is_canonical(const uint8_t* b, int len, bool compressed) {
   return o == 0;
 }
 
+// A point that fails is stored as infinity; its error bits (2 = bad encoding / off the curve, 4 = outside the subgroup) are
+// OR-ed into *err and, when `status` is given, written to status[i] (0 for a good point).
 struct G1DecodeK {
   static constexpr int BLOCK = 128;
-  PS_DEV static void run(uint32_t i, const uint8_t* in, int format, G1Affine* out, uint32_t* err, int subgroup) {
+  PS_DEV static void run(uint32_t i, const uint8_t* in, int format, G1Affine* out, uint32_t* err, int subgroup, uint8_t* status) {
     const uint8_t* b = in + (size_t)i * (format == PS_FMT_COMPRESSED ? 48 : 96);
     uint8_t flags = b[0];
     bool ok = true;
@@ -168,15 +170,18 @@ struct G1DecodeK {
         p = G1Affine{x, y};
       }
     }
-    if (!ok) { ps_atomic_or(err, 2u); p = G1Affine::inf(); }
-    else if (subgroup && !p.is_inf() && !in_subgroup(p)) { ps_atomic_or(err, 4u); p = G1Affine::inf(); }
+    uint32_t e = 0;
+    if (!ok) e = 2u;
+    else if (subgroup && !p.is_inf() && !in_subgroup(p)) e = 4u;
+    if (e) { ps_atomic_or(err, e); p = G1Affine::inf(); }
+    if (status) status[i] = (uint8_t)e;
     out[i] = p;
   }
 };
 
 struct G2DecodeK {
   static constexpr int BLOCK = 64;
-  PS_DEV static void run(uint32_t i, const uint8_t* in, int format, G2Affine* out, uint32_t* err, int subgroup) {
+  PS_DEV static void run(uint32_t i, const uint8_t* in, int format, G2Affine* out, uint32_t* err, int subgroup, uint8_t* status) {
     const uint8_t* b = in + (size_t)i * (format == PS_FMT_COMPRESSED ? 96 : 192);
     uint8_t flags = b[0];
     bool ok = true;
@@ -205,8 +210,11 @@ struct G2DecodeK {
         p = G2Affine{x, y};
       }
     }
-    if (!ok) { ps_atomic_or(err, 2u); p = G2Affine::inf(); }
-    else if (subgroup && !p.is_inf() && !in_subgroup(p)) { ps_atomic_or(err, 4u); p = G2Affine::inf(); }
+    uint32_t e = 0;
+    if (!ok) e = 2u;
+    else if (subgroup && !p.is_inf() && !in_subgroup(p)) e = 4u;
+    if (e) { ps_atomic_or(err, e); p = G2Affine::inf(); }
+    if (status) status[i] = (uint8_t)e;
     out[i] = p;
   }
 };

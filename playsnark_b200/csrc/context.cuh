@@ -41,6 +41,10 @@ struct ps_ctx {
   // phase events of the last Groth16 prove: start, quotient done, MSM A, MSM C, MSM B, encoded
   void* evp[6] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
   bool evp_valid = false;
+  // phase events of the last ps_g16_verify_batch: start, uploaded, decoded, weighted, io sums, Miller loops, tree, root
+  // check, bisection done
+  void* evv[9] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
+  bool evv_valid = false;
   // point decoding rejects points outside the prime-order subgroup (kilic's FromCompressed does); 0 skips the
   // r-multiplication for key material the caller vouches for
   int subgroup_check = 1;
@@ -70,6 +74,14 @@ inline int ctx_event(ps_ctx* ctx, int i) {
   if (!ctx->timing_events) return PS_OK;
 #if PS_GPU
   if (ctx->ev[i]) PS_CUDA_TRY(cudaEventRecord((cudaEvent_t)ctx->ev[i], ctx->stream));
+#else
+  (void)ctx; (void)i;
+#endif
+  return PS_OK;
+}
+inline int ctx_verify_event(ps_ctx* ctx, int i) {
+#if PS_GPU
+  if (ctx->evv[i]) PS_CUDA_TRY(cudaEventRecord((cudaEvent_t)ctx->evv[i], ctx->stream));
 #else
   (void)ctx; (void)i;
 #endif

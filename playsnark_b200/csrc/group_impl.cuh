@@ -113,9 +113,16 @@ int GroupOps<F>::msm_batch(ps_ctx* ctx, const MsmPlan& plan, const Affine<F>* sl
 }
 
 template <class F>
-int GroupOps<F>::decode(ps_ctx* ctx, const uint8_t* d_in, size_t n, int format, Affine<F>* d_out, uint32_t* d_err, bool subgroup_check) {
+int GroupOps<F>::decode(ps_ctx* ctx, const uint8_t* d_in, size_t n, int format, Affine<F>* d_out, uint32_t* d_err, bool subgroup_check,
+                        uint8_t* d_status) {
   using DK = typename DecodeKernel<F>::K;
-  PS_LAUNCH(DK, ctx->stream, n, d_in, format, d_out, d_err, subgroup_check ? 1 : 0);
+  PS_LAUNCH(DK, ctx->stream, n, d_in, format, d_out, d_err, subgroup_check ? 1 : 0, d_status);
+  return PS_OK;
+}
+
+template <class F>
+int GroupOps<F>::to_affine(ps_ctx* ctx, const XYZZ<F>* d_in, size_t n, Affine<F>* d_out) {
+  PS_LAUNCH(BatchToAffineK<F>, ctx->stream, (n + BatchToAffineK<F>::K - 1) / BatchToAffineK<F>::K, (uint32_t)n, d_in, d_out);
   return PS_OK;
 }
 

@@ -83,8 +83,12 @@ struct GroupOps {
   // output's table offset); results (XYZZ) to d_out[0..plan.nsets)
   static int msm_batch(ps_ctx* ctx, const MsmPlan& plan, const Affine<F>* slab, XYZZ<F>* d_out);
   // wire bytes (device) -> affine Montgomery points; *d_err |= 2 on a bad encoding / a point off the curve,
-  // |= 4 on a point outside the prime-order subgroup (checked when subgroup_check is set)
-  static int decode(ps_ctx* ctx, const uint8_t* d_in, size_t n, int format, Affine<F>* d_out, uint32_t* d_err, bool subgroup_check);
+  // |= 4 on a point outside the prime-order subgroup (checked when subgroup_check is set); d_status (optional) receives
+  // those bits per point, 0 for a good one
+  static int decode(ps_ctx* ctx, const uint8_t* d_in, size_t n, int format, Affine<F>* d_out, uint32_t* d_err, bool subgroup_check,
+                    uint8_t* d_status = nullptr);
+  // XYZZ -> affine, one field inversion per few points
+  static int to_affine(ps_ctx* ctx, const XYZZ<F>* d_in, size_t n, Affine<F>* d_out);
   // tables t = 1..T-1 of a base set: tab[t][i] = 2^(c t) tab[0][i]
   static int tables_finish(ps_ctx* ctx, Affine<F>* tab, size_t n, int c, int T);
   // out[i] = scalar[i] * generator (standard-form limbs on the device)

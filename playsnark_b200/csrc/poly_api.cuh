@@ -64,6 +64,10 @@ int g16_setup_scalars(ps_ctx* ctx, const ps_qap* q, const uint8_t* toxic_be, G16
 struct Phgr13SetupScalars { Fr* pw; Fr* ek[9]; Fr* consts; };
 int phgr13_setup_scalars(ps_ctx* ctx, const ps_qap* q, const uint8_t* toxic_be, Phgr13SetupScalars* o);
 
+// (capi.cu) `rows` G1 MSMs over all points of one base set, row k's scalars at d_scalars + k * b->n * 8 (limbs), result k to
+// d_out_xyzz[k]; MSM_MAX_SEG rows share one pipeline
+int msm_rows_g1(ps_ctx* ctx, const ps_bases* b, const uint32_t* d_scalars, size_t rows, int mont, void* d_out_xyzz);
+
 // host-only helpers shared by both translation units
 inline int parse_fr(const uint8_t* src, Fr* out) {   // 32 B big-endian, canonical -> Montgomery
   Fr x;

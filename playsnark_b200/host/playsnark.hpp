@@ -233,6 +233,29 @@ inline bool Groth16Verify(Backend& b, const Groth16VerifKey& vk, const Groth16Pr
                       p.A.data(), p.B.data(), p.C.data(), &ok));
   return ok == 1;
 }
+// Groth16Verify for many proofs against one key as ONE combined pairing-product check with random 128-bit weights drawn
+// by the library (ps_g16_verify_batch).  True iff every proof verifies; per_proof (optional) receives one verdict per proof.
+inline bool Groth16VerifyBatch(Backend& b, const Groth16VerifKey& vk, const std::vector<Groth16Proof>& proofs,
+                               const std::vector<Vector>& ios, std::vector<bool>* per_proof = nullptr) {
+  const size_t n = proofs.size(), n_io = vk.IoLP.size();
+  if (ios.size() != n) throw std::invalid_argument("different number of proofs than public input vectors");
+  Poly w;
+  w.reserve(n * n_io);
+  std::vector<G1> A, C;
+  std::vector<G2> B;
+  for (size_t i = 0; i < n; i++) {
+    if (ios[i].size() < n_io) throw std::invalid_argument("different number of public inputs than IoLP elements");
+    for (size_t j = 0; j < n_io; j++) w.push_back(ToFieldElement(ios[i][j]));
+    A.push_back(proofs[i].A); B.push_back(proofs[i].B); C.push_back(proofs[i].C);
+  }
+  auto iolp = flatten(vk.IoLP), wb = flatten(w), ab = flatten(A), bb = flatten(B), cb = flatten(C);
+  std::vector<uint8_t> verdicts(n);
+  int ok = 0;
+  check(ps_g16_verify_batch(b.ctx(), vk.Alpha.data(), vk.Beta2.data(), vk.Gamma.data(), vk.Delta2.data(), iolp.data(), n_io, n,
+                            wb.data(), ab.data(), bb.data(), cb.data(), nullptr, &ok, per_proof ? verdicts.data() : nullptr));
+  if (per_proof) per_proof->assign(verdicts.begin(), verdicts.end());
+  return ok == 1;
+}
 // PHGR13Verify, pinochio.go:281-375; vs / ws / ys = the commitments of the public variables (vk.vs[:diff] ...)
 struct PHGR13VerifKey {  // pinochio.go:66-90
   G2 av{}, ay{}, gamma{}, bgamma2{}, yts{};
