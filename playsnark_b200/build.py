@@ -111,6 +111,7 @@ def build_variant(name: str, flags, tus=("capi_poly.cu",)) -> str:
 
 TEST_BUILD = os.path.join(ROOT, "tests", "_build")
 DEVICE_HARNESS = os.path.join(ROOT, "tests", "device_arith.cu")
+PAIRING_HARNESS = os.path.join(ROOT, "tests", "device_pairing.cu")
 
 
 def can_write(dir_path: str) -> bool:
@@ -123,17 +124,27 @@ def can_write(dir_path: str) -> bool:
     return os.access(dir_path, os.W_OK | os.X_OK)
 
 
-def build_device_harness(out_dir: str = TEST_BUILD) -> str:
-    """TEST-ONLY: the field / group-law harness of the GPU suite (tests/device_arith.cu, loaded by
-    tests/test_gpu_arith.py) as out_dir/libdevice_arith.so for sm_100a, rebuilt when it or a header it includes
-    has changed.  Written under a temporary name and renamed, so a reader never loads a partial file."""
-    so = os.path.join(out_dir, "libdevice_arith.so")
-    if not stale(so, _deps(DEVICE_HARNESS)):
+def harness_path(out_dir: str = TEST_BUILD, source: str = DEVICE_HARNESS, host: bool = False) -> str:
+    """where build_device_harness puts `source`: out_dir/lib<name>.so (lib<name>_host.so for the host build)"""
+    name = os.path.basename(source).rsplit(".", 1)[0]
+    return os.path.join(out_dir, "lib%s%s.so" % (name, "_host" if host else ""))
+
+
+def build_device_harness(out_dir: str = TEST_BUILD, source: str = DEVICE_HARNESS, host: bool = False) -> str:
+    """TEST-ONLY: a device harness of the GPU suite (tests/device_arith.cu for tests/test_gpu_arith.py,
+    tests/device_pairing.cu for tests/test_gpu_pairing.py) as out_dir/lib<name>.so for sm_100a, rebuilt when it or a
+    header it includes has changed.  host=True compiles the same file with g++ -DPS_HOST_EMU instead (kernels become
+    serial loops, for the CPU suite) as lib<name>_host.so.  Written under a temporary name and renamed, so a reader
+    never loads a partial file."""
+    so = harness_path(out_dir, source, host)
+    if not stale(so, _deps(source)):
         return so
     os.makedirs(out_dir, exist_ok=True)
     tmp = "%s.%d.tmp" % (so, os.getpid())
-    nvcc = os.environ.get("NVCC", "nvcc")
-    cmd = [nvcc] + NVCC_FLAGS + ["-split-compile", "0", "-shared", "-o", tmp, DEVICE_HARNESS]
+    if host:
+        cmd = ["g++", "-O2", "-std=c++17", "-x", "c++", "-DPS_HOST_EMU", "-fPIC", "-shared", "-o", tmp, source]
+    else:
+        cmd = [os.environ.get("NVCC", "nvcc")] + NVCC_FLAGS + ["-split-compile", "0", "-shared", "-o", tmp, source]
     print("[playsnark_b200] " + " ".join(cmd), file=sys.stderr)
     try:
         subprocess.check_call(cmd, cwd=ROOT)
