@@ -98,6 +98,12 @@ int ps_bases_export(ps_ctx* ctx, const ps_bases* b, size_t first, size_t count, 
 /* n must equal ps_bases_len(b) (PS_ERR_LENGTH otherwise, like the reference's panic).
  * out: 48 B (G1) / 96 B (G2) compressed.                                                       */
 int ps_msm(ps_ctx* ctx, const ps_bases* b, const uint8_t* scalars_be, size_t n, uint8_t* out);
+/* `rows` MSMs against the same base set in one call (many BlindEvals against one resident key): scalars_be holds
+ * rows x n scalars, row-major; out[k] = sum_i scalars[k][i] * P[i], `rows` compressed points.  n must equal
+ * ps_bases_len(b) (PS_ERR_LENGTH otherwise).  All rows share one Pippenger pipeline (one bucket set per row), split
+ * into several only when one pipeline would pass 2^31 bucket entries.  A base set loaded with all window tables
+ * (precompute_tables = -1) is best given a window chosen for rows x n points and `rows` outputs.                  */
+int ps_msm_rows(ps_ctx* ctx, const ps_bases* b, const uint8_t* scalars_be, size_t n, size_t rows, uint8_t* out);
 /* Partial-range / device-resident variant for sharding and benchmarking: scalars already on the
  * device as 8 little-endian u32 limbs each, standard (non-Montgomery) form; sums bases
  * [first, first+n) and leaves the partial as an XYZZ point (4 field elements, Montgomery limbs)
@@ -280,6 +286,22 @@ int ps_g16_verify_batch(ps_ctx* ctx, const uint8_t* alpha, const uint8_t* beta2,
  * proof = the 432 bytes of ps_phgr13_prove.                                                                     */
 int ps_phgr13_verify(ps_ctx* ctx, const uint8_t* vk_fixed, const uint8_t* vs, const uint8_t* ws, const uint8_t* ys,
                      size_t n_io, const uint8_t* io_be, const uint8_t* proof, int* ok);
+/* PHGR13Verify for n_proofs proofs against one key as ONE combined pairing-product check.  Proof i gets five independent
+ * random nonzero 128-bit weights rho_i1..rho_i5, one per equation of pinochio.go:312-372, and the batch is accepted iff
+ *   prod_i e(rho1 gv_i, gw_i) * e(sum_i [rho2 vass_i + rho3 wass_i + rho4 yass_i - rho1 yss_i]
+ *                                 - sum_k (sum_i rho_i1 io_ik) ys_k, G2gen)
+ *   * e(-sum rho1 hs_i, yts) e(-sum rho2 vss_i, av) e(-sum rho4 yss_i, ay) e(sum rho5 gz_i, gamma)
+ *   * e(-sum rho5 (vss_i + yss_i), bgamma2) e(-aw, sum rho3 wss_i) e(-bgamma, sum rho5 wss_i) == 1
+ * with gv_i = sum_k io_ik vs_k + vss_i and gw_i = sum_k io_ik ws_k + wss_i: n_proofs + 8 Miller loops and one final
+ * exponentiation.  A batch with an invalid proof is accepted with probability <= 2^-128 over the weights.
+ *   vk_fixed, vs, ws, ys, n_io: as ps_phgr13_verify.  io_be: n_proofs x n_io x 32 bytes, proof-major.
+ *   proofs: n_proofs x 432 bytes, each in ps_phgr13_prove's order.
+ *   weights: NULL (drawn by the library: getrandom) or n_proofs x 5 x 16 bytes big-endian (tests).
+ *   *ok, per_proof, and the status codes: as ps_g16_verify_batch (all 8 points of every proof are checked for the
+ *   curve and the subgroup; a proof that fails is invalid and left out of the sums).                              */
+int ps_phgr13_verify_batch(ps_ctx* ctx, const uint8_t* vk_fixed, const uint8_t* vs, const uint8_t* ws, const uint8_t* ys,
+                           size_t n_io, size_t n_proofs, const uint8_t* io_be, const uint8_t* proofs,
+                           const uint8_t* weights, int* ok, uint8_t* per_proof);
 
 /* PHGR13Prove (pinochio.go:207-254).  out: hs, vss, yss, vass, wass, yass, gz (7 x 48 B, in this
  * order) then wss (96 B) = 432 bytes.                                                           */
@@ -346,9 +368,11 @@ int ps_last_msm_timing(ps_ctx* ctx, float out_ms[5]);
  * [1] MSMs A and C (G1, one batched pipeline), [2] 0 (kept for layout), [3] normalise + encode A and C, [4] what
  * then remains of MSM B and its encoding (G2, concurrently on a second stream), [5] total          */
 int ps_last_prove_timing(ps_ctx* ctx, float out_ms[6]);
-/* device time in ms of the last ps_g16_verify_batch, by phase: [0] upload of points and weights, [1] decode + subgroup
- * checks, [2] weighting (rho_i A_i, rho_i C_i), [3] upload + conversion of the io values, [4] the proofs' Miller loops, [5] tree of products and sums, [6] root check
- * (io sums + MSM, three Miller loops, final exponentiation), [7] bisection for the per-proof verdicts, [8] total      */
+/* device time in ms of the last batch verifier call (ps_g16_verify_batch or ps_phgr13_verify_batch), by phase:
+ * [0] upload of points and weights, [1] decode + subgroup checks, [2] weighting (Groth16: rho_i A_i, rho_i C_i;
+ * PHGR13: the weighted proof points), [3] upload + conversion of the io values (PHGR13: also the per-proof io MSMs
+ * of gv_i in G1 and gw_i in G2), [4] the proofs' Miller loops, [5] tree of products and sums, [6] root check (io sums
+ * + MSM, the fixed pairs' Miller loops, final exponentiation), [7] bisection for the per-proof verdicts, [8] total  */
 int ps_last_verify_batch_timing(ps_ctx* ctx, float out_ms[9]);
 
 #ifdef __cplusplus

@@ -7,6 +7,6 @@ sm_100a CUDA kernels (playsnark_b200/csrc).
 from .api import (  # noqa: F401
     MultiBackend, MultiBases, NewGroth16TrustedSetup, NewPHGR13TrustedSetup,
     R, Backend, Bases, HostBuffer, Groth16Proof, Groth16Setup, PHGR13EvalKey, PHGR13Proof, QAP, SparseQAP, R1CS, Groth16Prove,
-    PHGR13Prove, Quotient, BlindEval, ToQAP, default_backend, set_default_backend, Groth16Verify, Groth16VerifyBatch, PHGR13Verify, PairingCheckBatch,
+    PHGR13Prove, Quotient, BlindEval, ToQAP, default_backend, set_default_backend, Groth16Verify, Groth16VerifyBatch, PHGR13Verify, PHGR13VerifyBatch, PairingCheckBatch,
 )
 from ._lib import PlaysnarkError  # noqa: F401

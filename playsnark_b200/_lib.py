@@ -37,6 +37,7 @@ SYMBOLS = [
     ("ps_bases_from_scalars", _I, [_P, _I, _B, _SZ, _I, _I, C.POINTER(_P)]),
     ("ps_bases_export", _I, [_P, _P, _SZ, _SZ, _I, _P]),
     ("ps_msm", _I, [_P, _P, _P, _SZ, _P]),
+    ("ps_msm_rows", _I, [_P, _P, _P, _SZ, _SZ, _P]),
     ("ps_msm_device", _I, [_P, _P, _SZ, _P, _SZ, _P]),
     ("ps_msm_device_mont", _I, [_P, _P, _SZ, _P, _SZ, _P]),
     ("ps_msm_combine", _I, [_P, _I, _P, _SZ, _P]),
@@ -74,6 +75,7 @@ SYMBOLS = [
     ("ps_g16_verify", _I, [_P, _B, _B, _B, _B, _B, _SZ, _B, _B, _B, _B, C.POINTER(C.c_int)]),
     ("ps_g16_verify_batch", _I, [_P, _B, _B, _B, _B, _B, _SZ, _SZ, _P, _P, _P, _P, _P, C.POINTER(C.c_int), _P]),
     ("ps_phgr13_verify", _I, [_P, _B, _B, _B, _B, _SZ, _B, _B, C.POINTER(C.c_int)]),
+    ("ps_phgr13_verify_batch", _I, [_P, _B, _P, _P, _P, _SZ, _SZ, _P, _P, _P, C.POINTER(C.c_int), _P]),
     ("ps_mctx_create", _I, [C.POINTER(C.c_int), _I, C.POINTER(_P)]),
     ("ps_mctx_destroy", None, [_P]),
     ("ps_mctx_size", _I, [_P]),

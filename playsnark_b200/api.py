@@ -218,6 +218,23 @@ class Backend:
         self._check(st)
         return out.raw
 
+    def msm_rows(self, bases: Bases, scalars, rows: int) -> List[bytes]:
+        """`rows` MSMs against the same bases in one call (ps_msm_rows): `scalars` = rows x len(bases) values, row-major
+        (a flat list, a list of rows, or wire bytes); returns one compressed point per row."""
+        if not isinstance(scalars, (bytes, bytearray)) and len(scalars) and isinstance(scalars[0], (list, tuple)):
+            scalars = [v for row in scalars for v in row]
+        buf = scalars if isinstance(scalars, (bytes, bytearray)) else _fr_bytes(scalars)
+        if rows < 0 or (rows and len(buf) % (32 * rows)):
+            raise ValueError("scalars do not split into %d rows" % rows)
+        n = len(buf) // 32 // rows if rows else len(bases)
+        per = 48 if bases.group == L.PS_G1 else 96
+        out = C.create_string_buffer(max(1, rows * per))
+        st = self.lib.ps_msm_rows(self.ctx, bases.handle, bytes(buf) or None, n, rows, out)
+        if st == L.PS_ERR_LENGTH:
+            raise ValueError("mismatch of length between poly %d and blinded eval points %d" % (n, len(bases)))
+        self._check(st)
+        return [out.raw[k * per:(k + 1) * per] for k in range(rows)]
+
     def prove_timing(self):
         t = (C.c_float * 6)()
         self._check(self.lib.ps_last_prove_timing(self.ctx, t))
@@ -839,3 +856,47 @@ def PHGR13Verify(vk: dict, qap, p: PHGR13Proof, io: Vector, backend: Optional[Ba
                                     proof, C.byref(ok)))
     return ok.value == 1
 
+
+def PHGR13VerifyBatch(vk: dict, qap, proofs: Sequence[PHGR13Proof], ios, backend: Optional[Backend] = None,
+                      weights=None, per_proof: bool = False):
+    """PHGR13Verify for many proofs against one key, decided as ONE combined pairing-product check with five random
+    128-bit weights per proof, one per equation (ps_phgr13_verify_batch).  `vk` as PHGR13Verify's; `ios` = one
+    public-input vector per proof (each at least nbVars - nbIO long, like PHGR13Verify's `io`), or one wire-format blob /
+    HostBuffer of len(proofs) x (nbVars - nbIO) values, proof-major.  `weights` (tests only) = one 5-tuple of nonzero
+    integers below 2^128 per proof; by default the library draws them from the operating system.  Returns True iff every
+    proof verifies; with per_proof=True a list with one verdict per proof.  A proof whose points do not decode, or lie
+    outside the prime-order subgroup, is simply invalid."""
+    b = backend or default_backend()
+    n_io, n = qap.nbVars - qap.nbIO, len(proofs)
+    if isinstance(ios, (HostBuffer, bytes, bytearray, memoryview)):
+        nbytes = ios.nbytes if isinstance(ios, HostBuffer) else len(ios)
+        if nbytes != n * n_io * 32:
+            raise ValueError("different number of public inputs than verification-key elements")
+        io_arg = _fr_bytes(ios)
+    else:
+        if len(ios) != n:
+            raise ValueError("different number of proofs than public input vectors")
+        for io in ios:
+            if len(io) < n_io:
+                raise ValueError("different number of public inputs than verification-key elements")
+        io_arg = b"".join(_fr_bytes(list(io[:n_io])) for io in ios)
+    w_arg = None
+    if weights is not None:
+        if len(weights) != n or any(len(w) != 5 for w in weights):
+            raise ValueError("five weights per proof")
+        if any(not 0 < int(x) < 1 << 128 for w in weights for x in w):
+            raise ValueError("weights must be nonzero 128-bit integers")
+        w_arg = b"".join(int(x).to_bytes(16, "big") for w in weights for x in w)
+    fixed = vk["av"] + vk["aw"] + vk["ay"] + vk["gamma"] + vk["bgamma"] + vk["bgamma2"] + vk["yts"]
+    blob = b"".join(p.hs + p.vss + p.yss + p.vass + p.wass + p.yass + p.gz + p.wss for p in proofs)
+    j = lambda xs: b"".join(xs[:n_io]) or None
+    ok = C.c_int(0)
+    verdicts = C.create_string_buffer(max(1, n)) if per_proof else None
+    st = b.lib.ps_phgr13_verify_batch(b.ctx, fixed, j(vk["vs"]), j(vk["ws"]), j(vk["ys"]), n_io, n, io_arg or None, blob or None,
+                                      w_arg, C.byref(ok), verdicts)
+    if st == L.PS_ERR_ARG and weights is not None:
+        raise ValueError("weights must be nonzero 128-bit integers")
+    b._check(st)
+    if per_proof:
+        return [verdicts.raw[i] == 1 for i in range(n)]
+    return ok.value == 1

@@ -8,6 +8,7 @@
 #include "microbench.cuh"
 #include "multi_api.cuh"
 
+#include <algorithm>
 #include <new>
 
 using namespace ps;
@@ -222,21 +223,6 @@ int bases_concat_into(ps_ctx* ctx, ps_bases* b, int format, const uint8_t* const
   return bases_fill_t<F>(ctx, b, buf.data(), format);
 }
 
-// window of a batch of `nsets` MSMs over `total_points` points in all (per shard): every set pays its own bucket
-// merge + reduction, the mixed additions are shared (same model as msm_pick_window_full, which is the case nsets = 1)
-int batch_window(ps_ctx* ctx, size_t total_points, int nsets) {
-  const size_t shards = (size_t)(ctx->msm_shards > 0 ? ctx->msm_shards : 1);
-  const double n = (double)(total_points / shards + 1), bucket_cost = (double)ctx->msm_bucket_cost * (nsets > 0 ? nsets : 1);
-  int best = 4; double best_cost = 1e300;
-  for (int c = 4; c <= 24; c++) {
-    double W = msm_windows(c);
-    if (n * W >= 2.0e9) continue;
-    double cost = n * W * 10.0 + (double)(1u << (c - 1)) * bucket_cost;
-    if (cost < best_cost) { best_cost = cost; best = c; }
-  }
-  return best;
-}
-
 // allocates the three base sets of a Groth16 key: A and C carved out of one G1 slab, B (G2) on its own
 int g16_key_alloc(ps_g16_key* k, size_t nA, size_t nB, size_t nC, int window_g1, int window_g2) {
   const size_t g1counts[2] = {nA, nC};
@@ -263,17 +249,48 @@ int phgr13_key_alloc(ps_ctx* ctx, ps_phgr13_key* k, size_t n_gates, size_t n_mid
 }  // namespace
 
 namespace ps {
-int msm_rows_g1(ps_ctx* ctx, const ps_bases* b, const uint32_t* d_scalars, size_t rows, int mont, void* d_out_xyzz) {
-  if (!b || b->group != PS_G1) return PS_ERR_ARG;
-  G1XYZZ* out = (G1XYZZ*)d_out_xyzz;
-  for (size_t r0 = 0; r0 < rows; r0 += MSM_MAX_SEG) {
-    const int cnt = (int)(rows - r0 < (size_t)MSM_MAX_SEG ? rows - r0 : (size_t)MSM_MAX_SEG);
-    SegSpec sg[MSM_MAX_SEG];
-    for (int k = 0; k < cnt; k++) sg[k] = SegSpec{b, 0, d_scalars + (r0 + k) * b->n * 8, b->n, mont, k};
-    PS_TRY(msm_batch<Fp>(ctx, sg, cnt, cnt, out + r0));
+// window of a batch of `nsets` MSMs over `total_points` points in all (per shard): every set pays its own bucket
+// merge + reduction, the mixed additions are shared (same model as msm_pick_window_full, which is the case nsets = 1)
+int batch_window(ps_ctx* ctx, size_t total_points, int nsets) {
+  const size_t shards = (size_t)(ctx->msm_shards > 0 ? ctx->msm_shards : 1);
+  const double n = (double)(total_points / shards + 1), bucket_cost = (double)ctx->msm_bucket_cost * (nsets > 0 ? nsets : 1);
+  int best = 4; double best_cost = 1e300;
+  for (int c = 4; c <= 24; c++) {
+    double W = msm_windows(c);
+    if (n * W >= 2.0e9) continue;
+    double cost = n * W * 10.0 + (double)(1u << (c - 1)) * bucket_cost;
+    if (cost < best_cost) { best_cost = cost; best = c; }
+  }
+  return best;
+}
+
+template <class F>
+int msm_rows(ps_ctx* ctx, const ps_bases* b, const uint32_t* d_scalars, size_t rows, int mont, XYZZ<F>* d_out) {
+  if (!b || b->group != PointBytes<F>::GROUP) return PS_ERR_ARG;
+  if (rows == 0) return PS_OK;
+  const size_t n = b->n;
+  if (n == 0) return dev_memset(d_out, 0, rows * sizeof(XYZZ<F>), ctx->stream);
+  // every row has its own bucket sets, so a window without precomputed tables is chosen as for one row
+  const int c = b->c ? b->c : msm_pick_window(n), W = msm_windows(c), T = b->T, S = (W + T - 1) / T;
+  // rows per pipeline: entry positions and bucket indices of one pipeline stay below 2^31
+  const size_t lim = 0x7FFFFFFFull, per = std::max((size_t)n * W, (size_t)S << (c - 1));
+  if (per > lim) return PS_ERR_UNSUPPORTED;
+  const size_t cap = lim / per;
+  for (size_t r0 = 0; r0 < rows; r0 += cap) {
+    const size_t cnt = std::min(cap, rows - r0);
+    MsmPlan p;
+    memset(&p, 0, sizeof p);
+    p.c = c; p.W = W; p.T = T; p.S = S; p.D = 1u << (c - 1);
+    p.total = (uint32_t)(cnt * n); p.nseg = 1; p.nsets = (int)cnt; p.row_len = (uint32_t)n;
+    p.seg[0].scalars = d_scalars + r0 * n * 8; p.seg[0].n = p.total; p.seg[0].mont = (uint32_t)mont;
+    p.nbase[0] = (uint32_t)n;
+    p.toff[0] = (uint32_t)(((const char*)b->tab - (const char*)b->slab) / sizeof(Affine<F>));
+    PS_TRY(GroupOps<F>::msm_batch(ctx, p, (const Affine<F>*)b->slab, d_out + r0));
   }
   return PS_OK;
 }
+template int msm_rows<Fp>(ps_ctx*, const ps_bases*, const uint32_t*, size_t, int, XYZZ<Fp>*);
+template int msm_rows<Fp2>(ps_ctx*, const ps_bases*, const uint32_t*, size_t, int, XYZZ<Fp2>*);
 }  // namespace ps
 
 extern "C" {
@@ -512,6 +529,28 @@ int ps_msm(ps_ctx* ctx, const ps_bases* b, const uint8_t* scalars_be, size_t n, 
     if (!d_res) return PS_ERR_ALLOC;
     PS_TRY(msm_on_bases<Fp2>(ctx, b, 0, d_sc, n, 0, d_res));
     PS_TRY(encode_points<Fp2>(ctx, d_res, 1, out));
+  }
+  return check_err_flag(ctx, d_err, PS_ERR_ENCODING);
+}
+
+int ps_msm_rows(ps_ctx* ctx, const ps_bases* b, const uint8_t* scalars_be, size_t n, size_t rows, uint8_t* out) {
+  if (!b || (rows && !out) || (rows && n && !scalars_be)) return PS_ERR_ARG;
+  if (n != b->n) return PS_ERR_LENGTH;
+  if (n && rows > ((size_t)1 << 40) / n) return PS_ERR_UNSUPPORTED;
+  PS_TRY(begin_call(ctx));
+  if (rows == 0) return PS_OK;
+  uint32_t *d_sc = nullptr, *d_err = nullptr;
+  PS_TRY(stage_scalars(ctx, scalars_be, rows * n, 0, &d_sc, &d_err));
+  if (b->group == PS_G1) {
+    G1XYZZ* d_res = ctx->arena.take<G1XYZZ>(rows);
+    if (!d_res) return PS_ERR_ALLOC;
+    PS_TRY(msm_rows<Fp>(ctx, b, d_sc, rows, 0, d_res));
+    PS_TRY(encode_points<Fp>(ctx, d_res, rows, out));
+  } else {
+    G2XYZZ* d_res = ctx->arena.take<G2XYZZ>(rows);
+    if (!d_res) return PS_ERR_ALLOC;
+    PS_TRY(msm_rows<Fp2>(ctx, b, d_sc, rows, 0, d_res));
+    PS_TRY(encode_points<Fp2>(ctx, d_res, rows, out));
   }
   return check_err_flag(ctx, d_err, PS_ERR_ENCODING);
 }

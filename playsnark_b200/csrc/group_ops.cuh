@@ -35,6 +35,10 @@ struct MsmPlan {
   uint32_t D;      // buckets per set = 2^(c-1)
   uint32_t total;  // scalars in the batch
   int nseg, nsets;
+  // 0: segment mode (above).  Otherwise ROW mode: many MSMs of row_len scalars each against the same points of one base
+  // set -- seg[0] holds the scalars of all rows, contiguous and row-major; scalar i goes to output i / row_len and point
+  // seg[0].first + i % row_len; nbase[0] / toff[0] describe the base set; nsets = rows, not bounded by MSM_MAX_SEG
+  uint32_t row_len;
   MsmSeg seg[MSM_MAX_SEG];
   uint32_t nbase[MSM_MAX_SEG];  // per output: points per table (table stride)
   uint32_t toff[MSM_MAX_SEG];   // per output: offset (in points) of its first table inside the slab all outputs share

@@ -34,6 +34,27 @@ PS_DEV int msm_seg_of(const MsmPlan& p, uint32_t i) {
   return k;
 }
 
+// Where scalar i of the batch comes from and goes to: its scalar array and index in it, the first bucket of its output
+// set, the point it multiplies (offset in the slab) and the table stride of that base set.
+struct MsmSrc {
+  const uint32_t* scalars;
+  uint32_t idx, b0, pt, nbase;
+  int mont;
+};
+PS_DEV MsmSrc msm_source(const MsmPlan& p, uint32_t i) {
+  MsmSrc s;
+  if (p.row_len) {
+    const uint32_t set = i / p.row_len;
+    s.scalars = p.seg[0].scalars; s.idx = i; s.mont = (int)p.seg[0].mont;
+    s.b0 = set * (uint32_t)p.S * p.D; s.nbase = p.nbase[0]; s.pt = p.toff[0] + p.seg[0].first + (i - set * p.row_len);
+  } else {
+    const MsmSeg sg = p.seg[msm_seg_of(p, i)];
+    s.scalars = sg.scalars; s.idx = i - sg.start; s.mont = (int)sg.mont;
+    s.b0 = sg.set * (uint32_t)p.S * p.D; s.nbase = p.nbase[sg.set]; s.pt = p.toff[sg.set] + sg.first + s.idx;
+  }
+  return s;
+}
+
 // Loads scalar i (8 LE limbs), optionally leaves Montgomery form, folds k > (r-1)/2 to r-k.
 PS_DEV void msm_load_scalar(const uint32_t* scalars, uint32_t i, int mont, uint32_t k[8], bool& neg) {
   Fr x;
@@ -79,16 +100,15 @@ PS_DEV bool msm_next_digit(uint32_t k[8], int c, uint32_t& carry, uint32_t& mag,
 struct MsmCountK {
   static constexpr int BLOCK = 256;
   PS_DEV static void run(uint32_t i, MsmPlan p, uint32_t* count, uint32_t* ranks) {
-    const MsmSeg sg = p.seg[msm_seg_of(p, i)];
+    const MsmSrc src = msm_source(p, i);
     uint32_t k[8]; bool neg;
-    msm_load_scalar(sg.scalars, i - sg.start, (int)sg.mont, k, neg);
+    msm_load_scalar(src.scalars, src.idx, src.mont, k, neg);
     uint32_t carry = 0;
-    const uint32_t b0 = sg.set * (uint32_t)p.S * p.D;
     for (int w = 0; w < p.W; w++) {
       uint32_t mag; bool dneg;
       uint32_t rank = 0xFFFFFFFFu;
       if (msm_next_digit(k, p.c, carry, mag, dneg)) {
-        uint32_t b = b0 + (uint32_t)(w / p.T) * p.D + (mag - 1);
+        uint32_t b = src.b0 + (uint32_t)(w / p.T) * p.D + (mag - 1);
         rank = ps_atomic_add(count + b, 1u);
       }
       ranks[(size_t)w * p.total + i] = rank;
@@ -99,17 +119,16 @@ struct MsmCountK {
 struct MsmScatterK {
   static constexpr int BLOCK = 256;
   PS_DEV static void run(uint32_t i, MsmPlan p, const uint32_t* off, const uint32_t* ranks, uint32_t* ent) {
-    const MsmSeg sg = p.seg[msm_seg_of(p, i)];
+    const MsmSrc src = msm_source(p, i);
     uint32_t k[8]; bool neg;
-    msm_load_scalar(sg.scalars, i - sg.start, (int)sg.mont, k, neg);
+    msm_load_scalar(src.scalars, src.idx, src.mont, k, neg);
     uint32_t carry = 0;
-    const uint32_t b0 = sg.set * (uint32_t)p.S * p.D, nbase = p.nbase[sg.set], pt = p.toff[sg.set] + sg.first + (i - sg.start);
     for (int w = 0; w < p.W; w++) {
       uint32_t mag; bool dneg;
       if (msm_next_digit(k, p.c, carry, mag, dneg)) {
-        uint32_t b = b0 + (uint32_t)(w / p.T) * p.D + (mag - 1);
+        uint32_t b = src.b0 + (uint32_t)(w / p.T) * p.D + (mag - 1);
         uint32_t pos = off[b] + ranks[(size_t)w * p.total + i];
-        uint32_t idx = (uint32_t)(w % p.T) * nbase + pt;
+        uint32_t idx = (uint32_t)(w % p.T) * src.nbase + src.pt;
         ent[pos] = idx | ((neg != dneg) ? 0x80000000u : 0u);
       }
     }
@@ -552,19 +571,18 @@ static __global__ void __launch_bounds__(SCATTER2_BLOCK) k_scatter_stage(MsmPlan
 #pragma unroll
   for (int w = 0; w < SCATTER2_WMAX; w++) pos[w] = 0xFFFFFFFFu;
   if (i < p.total) {
-    const MsmSeg sg = p.seg[msm_seg_of(p, i)];
+    const MsmSrc src = msm_source(p, i);
     uint32_t k[8]; bool neg;
-    msm_load_scalar(sg.scalars, i - sg.start, (int)sg.mont, k, neg);
+    msm_load_scalar(src.scalars, src.idx, src.mont, k, neg);
     uint32_t carry = 0;
-    const uint32_t b0 = sg.set * (uint32_t)p.S * p.D, nbase = p.nbase[sg.set], pt = p.toff[sg.set] + sg.first + (i - sg.start);
 #pragma unroll
     for (int w = 0; w < SCATTER2_WMAX; w++) {
       if (w < p.W) {
         uint32_t mag; bool dneg;
         if (msm_next_digit(k, p.c, carry, mag, dneg)) {
-          const uint32_t b = b0 + (uint32_t)(w / p.T) * p.D + (mag - 1);
+          const uint32_t b = src.b0 + (uint32_t)(w / p.T) * p.D + (mag - 1);
           pos[w] = off[b] + ranks[(size_t)w * p.total + i];
-          val[w] = ((uint32_t)(w % p.T) * nbase + pt) | ((neg != dneg) ? 0x80000000u : 0u);
+          val[w] = ((uint32_t)(w % p.T) * src.nbase + src.pt) | ((neg != dneg) ? 0x80000000u : 0u);
           lr[w] = atomicAdd(&hist[pos[w] >> shift], 1u);
         }
       }
@@ -595,20 +613,19 @@ inline int scatter_stage(ps_stream_t st, const MsmPlan& p, const uint32_t* off, 
 #else
   (void)st; (void)nparts;
   for (uint32_t i = 0; i < p.total; i++) {
-    const MsmSeg sg = p.seg[msm_seg_of(p, i)];
+    const MsmSrc src = msm_source(p, i);
     uint32_t k[8]; bool neg;
-    msm_load_scalar(sg.scalars, i - sg.start, (int)sg.mont, k, neg);
+    msm_load_scalar(src.scalars, src.idx, src.mont, k, neg);
     uint32_t carry = 0;
-    const uint32_t b0 = sg.set * (uint32_t)p.S * p.D, nbase = p.nbase[sg.set], pt = p.toff[sg.set] + sg.first + (i - sg.start);
     for (int w = 0; w < p.W; w++) {
       uint32_t mag; bool dneg;
       if (!msm_next_digit(k, p.c, carry, mag, dneg)) continue;
-      const uint32_t b = b0 + (uint32_t)(w / p.T) * p.D + (mag - 1);
+      const uint32_t b = src.b0 + (uint32_t)(w / p.T) * p.D + (mag - 1);
       const uint32_t pos = off[b] + ranks[(size_t)w * p.total + i];
       const uint32_t part = pos >> shift;
       const size_t slot = ((size_t)part << shift) + part_count[part]++;
       staging[2 * slot] = pos;
-      staging[2 * slot + 1] = ((uint32_t)(w % p.T) * nbase + pt) | ((neg != dneg) ? 0x80000000u : 0u);
+      staging[2 * slot + 1] = ((uint32_t)(w % p.T) * src.nbase + src.pt) | ((neg != dneg) ? 0x80000000u : 0u);
     }
   }
 #endif
@@ -647,7 +664,8 @@ template <class F>
 int msm_run_batch(ps_ctx* ctx, const MsmPlan& g, const Affine<F>* tab, XYZZ<F>* d_out) {
   ps_stream_t st = ctx->stream;
   Arena& ar = ctx->arena;
-  if (g.nsets < 1 || g.nsets > MSM_MAX_SEG || g.nseg < 0 || g.nseg > MSM_MAX_SEG) return PS_ERR_ARG;
+  if (g.nsets < 1 || (g.nsets > MSM_MAX_SEG && !g.row_len) || g.nseg < 0 || g.nseg > MSM_MAX_SEG) return PS_ERR_ARG;
+  if (g.row_len && (g.nseg != 1 || (uint64_t)g.nsets * g.row_len != g.total)) return PS_ERR_ARG;
   if (g.total == 0) return dev_memset(d_out, 0, (size_t)g.nsets * sizeof(XYZZ<F>), st);
   const int S_all = g.nsets * g.S;                 // bucket sets of the whole batch
   const uint32_t nb = (uint32_t)S_all * g.D;

@@ -64,9 +64,13 @@ int g16_setup_scalars(ps_ctx* ctx, const ps_qap* q, const uint8_t* toxic_be, G16
 struct Phgr13SetupScalars { Fr* pw; Fr* ek[9]; Fr* consts; };
 int phgr13_setup_scalars(ps_ctx* ctx, const ps_qap* q, const uint8_t* toxic_be, Phgr13SetupScalars* o);
 
-// (capi.cu) `rows` G1 MSMs over all points of one base set, row k's scalars at d_scalars + k * b->n * 8 (limbs), result k to
-// d_out_xyzz[k]; MSM_MAX_SEG rows share one pipeline
-int msm_rows_g1(ps_ctx* ctx, const ps_bases* b, const uint32_t* d_scalars, size_t rows, int mont, void* d_out_xyzz);
+// (capi.cu) `rows` MSMs over all points of one base set of group F (Fp: G1, Fp2: G2), row k's scalars at
+// d_scalars + k * b->n * 8 (limbs), result k to d_out[k]; all rows run as one pipeline (MsmPlan's row mode), split into
+// several only where one pipeline's entry or bucket count would reach 2^31
+template <class F> struct XYZZ;
+template <class F> int msm_rows(ps_ctx* ctx, const ps_bases* b, const uint32_t* d_scalars, size_t rows, int mont, XYZZ<F>* d_out);
+// (capi.cu) window of a batch of `nsets` MSMs over `total_points` points in all, for base sets with all window tables
+int batch_window(ps_ctx* ctx, size_t total_points, int nsets);
 
 // host-only helpers shared by both translation units
 inline int parse_fr(const uint8_t* src, Fr* out) {   // 32 B big-endian, canonical -> Montgomery

@@ -5,6 +5,7 @@
 //   Groth16Prove(tr, q, sol)        groth16.go:122     PHGR13Prove(ek, qap, solution)  pinochio.go:207
 //   QAP::Quotient(sol)              qap.go:151         BlindEval(p, blindedPoint)      algebra.go:348
 //   Groth16Verify(vk, p, io)        groth16.go:214     PHGR13Verify(vk, p, io)         pinochio.go:281
+//   Groth16VerifyBatch / PHGR13VerifyBatch: many proofs against one key in one combined pairing check
 // Scalars are 32-byte big-endian Elements (kyber Scalar.MarshalBinary), points their compressed
 // MarshalBinary bytes.  Go panics become C++ exceptions with the same message.  No arithmetic lives
 // here: everything is computed by libplaysnark_b200.so on the GPU.
@@ -279,6 +280,37 @@ inline bool PHGR13Verify(Backend& b, const PHGR13VerifKey& vk, const PHGR13Proof
   auto vs = flatten(vk.vs), ws = flatten(vk.ws), ys = flatten(vk.ys), wb = flatten(w);
   int ok = 0;
   check(ps_phgr13_verify(b.ctx(), fixed, vs.data(), ws.data(), ys.data(), diff, wb.data(), proof, &ok));
+  return ok == 1;
+}
+// PHGR13Verify for many proofs against one key in one combined pairing check (ps_phgr13_verify_batch, weights drawn by
+// the library); per_proof (optional) receives one verdict per proof
+inline bool PHGR13VerifyBatch(Backend& b, const PHGR13VerifKey& vk, const std::vector<PHGR13Proof>& proofs,
+                              const std::vector<Vector>& ios, std::vector<bool>* per_proof = nullptr) {
+  const size_t n = proofs.size(), diff = vk.vs.size();
+  if (vk.ws.size() != diff || vk.ys.size() != diff)
+    throw std::invalid_argument("different number of public inputs than verification-key elements");
+  if (ios.size() != n) throw std::invalid_argument("different number of proofs than public input vectors");
+  uint8_t fixed[576];
+  std::memcpy(fixed, vk.av.data(), 96); std::memcpy(fixed + 96, vk.aw.data(), 48); std::memcpy(fixed + 144, vk.ay.data(), 96);
+  std::memcpy(fixed + 240, vk.gamma.data(), 96); std::memcpy(fixed + 336, vk.bgamma.data(), 48);
+  std::memcpy(fixed + 384, vk.bgamma2.data(), 96); std::memcpy(fixed + 480, vk.yts.data(), 96);
+  std::vector<uint8_t> blob(432 * n);
+  Poly w;
+  w.reserve(n * diff);
+  for (size_t i = 0; i < n; i++) {
+    if (ios[i].size() < diff) throw std::invalid_argument("different number of public inputs than verification-key elements");
+    for (size_t j = 0; j < diff; j++) w.push_back(ToFieldElement(ios[i][j]));
+    const PHGR13Proof& p = proofs[i];
+    const G1* order[7] = {&p.hs, &p.vss, &p.yss, &p.vass, &p.wass, &p.yass, &p.gz};
+    for (int k = 0; k < 7; k++) std::memcpy(blob.data() + 432 * i + 48 * k, order[k]->data(), 48);
+    std::memcpy(blob.data() + 432 * i + 336, p.wss.data(), 96);
+  }
+  auto vs = flatten(vk.vs), ws = flatten(vk.ws), ys = flatten(vk.ys), wb = flatten(w);
+  std::vector<uint8_t> verdicts(n);
+  int ok = 0;
+  check(ps_phgr13_verify_batch(b.ctx(), fixed, vs.data(), ws.data(), ys.data(), diff, n, wb.data(), blob.data(), nullptr, &ok,
+                               per_proof ? verdicts.data() : nullptr));
+  if (per_proof) per_proof->assign(verdicts.begin(), verdicts.end());
   return ok == 1;
 }
 
