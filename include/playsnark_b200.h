@@ -62,8 +62,8 @@ int ps_ctx_set_stream(ps_ctx* ctx, void* cuda_stream);
  * (one per GPU, ps_msm_device / ps_g16_msm_partials), so their automatic window is sized for n / N points;
  * "msm_bucket_cost" = cost of one bucket (merge + reduction) in the automatic window choice, in field
  * products with a mixed addition counting 10 (default 70, fitted on B200);
- * "msm_scatter" = 0 (one-pass scatter of the counting sort) | 1 (two passes through a partitioned staging
- * array when the entry array exceeds L2) | 2 (two passes whenever the window count allows; tests);
+ * "msm_scatter" = 0 (one-pass counting sort of the bucket entries) | 1 (two-level sort, by partition of buckets and
+ * then by bucket, from 2^25 entries n*W; default) | 2 (two-level sort whenever the bucket count allows; tests);
  * "msm_wave_floor" = 1 (short accumulate chunks: whole waves with the wave count rounded down, default) | 0 (rounded up);
  * "interp_fused" = 1 (lowest nine levels of the interpolation tree in one shared-memory kernel, default) | 0 (level by
  * level; identical coefficients).  Environment: PLAYSNARK_B200_STREAM2_PRIO=0 creates the secondary stream (G2 sums) at

@@ -56,8 +56,8 @@ struct ps_ctx {
   int msm_team = 1;
   // base sets loaded from now on are meant to be summed in this many index ranges (sharded proofs)
   int msm_shards = 1;
-  // counting-sort scatter: 0 = one pass, 1 = two passes through a partitioned staging array when the
-  // entry array exceeds L2 (msm.cuh), 2 = two passes whenever possible (tests)
+  // bucket sort of the MSM entries: 0 = one-pass counting sort, 1 = two-level sort from 2^25 entries (msm.cuh),
+  // 2 = two-level sort whenever possible (tests)
   int msm_scatter = PS_SCATTER_DEFAULT;
   // window model: time of one bucket (merge + reduction) in field products, a mixed addition being 10
   int msm_bucket_cost = PS_BUCKET_COST;
